@@ -415,6 +415,34 @@ def busy_intervals_ms(prof, base):
     return busy
 
 
+DUMP_SAMPLE = 1 << 17        # parameters kept per layer: 50 GPT-2-XL layers x 512 KiB = 25 MiB
+
+
+def dump_outputs(directory: str, engine):
+    """What the timed step hands its caller, as float32 / float64 .npy files: the engine's running total loss (a sum over
+    every micro-batch since the engine started; the engine never resets it) on the last stage, and for every layer a
+    fixed sample of its updated parameters (the optimizer step has already zeroed the gradients).  The sample of layer
+    ``i`` is the same ``DUMP_SAMPLE`` sorted positions in every run (seed ``i``), so that two builds can be compared
+    value for value.  Two runs of one build do not agree bit for bit, because the token-embedding gradient is
+    accumulated with floating-point atomics; on one B200 at a 1000 W power limit (GPT-2-XL, --steps 3 --warmup 2)
+    the parameters differed by at most 6e-7 of the layer's largest value.  Only the first pipeline writes: after the
+    all-reduce every replica holds the same layers."""
+    import numpy as np
+    pipeline = engine._pipeline
+    if pipeline._pipeline_id != 0:
+        return
+    os.makedirs(directory, exist_ok=True)
+    if pipeline.is_last_stage():
+        np.save(os.path.join(directory, "total_loss.npy"),
+                np.asarray(pipeline.execution.total_loss.detach().item(), dtype=np.float64))
+    for layer in pipeline.execution._layers:
+        n = layer.flat_param.numel()
+        idx = np.sort(np.random.default_rng(layer.layer_id).choice(n, size=min(n, DUMP_SAMPLE), replace=False))
+        idx = torch.from_numpy(idx).to(layer.flat_param.device)
+        np.save(os.path.join(directory, f"layer{layer.layer_id:03d}_param.npy"),
+                layer.flat_param.detach()[idx].float().cpu().numpy())
+
+
 def run_ours(args, cfg):
     import torch.distributed as dist
 
@@ -509,6 +537,8 @@ def run_ours(args, cfg):
     launches = L.load().oob_launch_count() - launches0
     g_ms, g_fl, g_ex, g_n = C.c_double(), C.c_double(), C.c_double(), C.c_long()
     L.call("oob_gemm_timing_end", C.byref(g_ms), C.byref(g_fl), C.byref(g_ex), C.byref(g_n))
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, engine)
     ms_e2e, losses = timed(args.steps, False, True)
 
     # one more (untimed) step with CUDA events around every forward / backward pass: how busy was each stage?
@@ -767,6 +797,9 @@ def main():
     ap.add_argument("--with-reconfig", type=int, default=int(os.environ.get("OOB_BENCH_RECONFIG", "1")), choices=[0, 1],
                     help="N >= 4: after the timed region, also kill a rank of a fresh job on the same GPUs and report "
                          "the recovery time under \"reconfiguration\" (adds 2-3 minutes)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed (loss and a fixed sample of every "
+                         "layer's parameters) to DIR/<name>.npy")
     ap.add_argument("--reconfig", action="store_true",
                     help="reconfiguration latency after a real kill of one rank (spawns its own workers; see "
                          "tools/reconfig_bench.py)")

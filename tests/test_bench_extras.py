@@ -118,3 +118,34 @@ def test_config4_line_is_condensed(monkeypatch):
     assert cmd[cmd.index("--with-reconfig") + 1] == "0"           # the embedded run never embeds another one
     assert out["value"] == 1.7e6 and out["config"]["parallelism"] == "dp2 x pp4" and out["parity_check"]["ok"]
     assert out["stage_layers"] == [5, 4, 4, 1] and "roofline" not in out and out["wall_s"] >= 0
+
+
+def test_dump_outputs_writes_the_same_sample_of_every_layer(tmp_path):
+    import types
+
+    import numpy as np
+    import torch
+
+    def layer(lid, n):
+        return types.SimpleNamespace(layer_id=lid, flat_param=torch.arange(n, dtype=torch.float32) * (lid + 1))
+
+    def engine(pipeline_id, layers):
+        execution = types.SimpleNamespace(_layers=layers, total_loss=torch.tensor(3.25))
+        return types.SimpleNamespace(_pipeline=types.SimpleNamespace(_pipeline_id=pipeline_id, execution=execution,
+                                                                     is_last_stage=lambda: True))
+
+    big = bench.DUMP_SAMPLE * 3
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), engine(0, [layer(0, 100), layer(7, big)]))
+    names = sorted(os.listdir(tmp_path / "a"))
+    assert names == ["layer000_param.npy", "layer007_param.npy", "total_loss.npy"]
+    for n in names:
+        a, b = np.load(tmp_path / "a" / n), np.load(tmp_path / "b" / n)
+        assert a.dtype in (np.float32, np.float64) and np.array_equal(a, b)
+    assert np.load(tmp_path / "a" / "total_loss.npy") == 3.25
+    assert np.array_equal(np.load(tmp_path / "a" / "layer000_param.npy"), np.arange(100, dtype=np.float32))
+    sample = np.load(tmp_path / "a" / "layer007_param.npy")
+    assert sample.shape == (bench.DUMP_SAMPLE,) and len(np.unique(sample)) == bench.DUMP_SAMPLE
+    assert np.all(sample[1:] > sample[:-1]) and np.all(sample % 8 == 0)    # sorted positions of layer 7's values
+    bench.dump_outputs(str(tmp_path / "c"), engine(1, [layer(0, 100)]))    # a second replica holds the same layers
+    assert not (tmp_path / "c").exists()

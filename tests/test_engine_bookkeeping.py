@@ -233,18 +233,13 @@ _LIVE = {}
 
 
 def live_reference_run():
-    """ONE child process that drives the reference's own classes (tests/golden/gen_golden.py --live: its Python from
-    /root/reference, its C++ planner objects when oracle/_ref is built) on fresh random inputs; shared by the tests below."""
-    import subprocess
-    import sys
-    if not os.path.isdir("/root/reference/oobleck"):
-        pytest.skip("needs /root/reference")
+    """What the reference's own classes produced on random inputs beyond the committed tables, shared by the tests below:
+    tests/golden/live_reference.json.gz, recorded by ``gen_golden.py --live 20260923 80 150 13`` (its Python, its C++
+    planner objects from oracle/_ref; the last stdout line, gzipped)."""
+    import gzip
     if "data" not in _LIVE:
-        r = subprocess.run([sys.executable, os.path.join(G, "gen_golden.py"), "--live", "20260923", "80", "150", "13"],
-                           capture_output=True, text=True, timeout=900)
-        line = next((l for l in reversed(r.stdout.splitlines()) if l.startswith('{"dp_groups"')), None)
-        assert r.returncode == 0 and line is not None, r.stderr[-2000:]
-        _LIVE["data"] = json.loads(line)
+        with gzip.open(os.path.join(G, "live_reference.json.gz"), "rt") as f:
+            _LIVE["data"] = json.load(f)
     return _LIVE["data"]
 
 

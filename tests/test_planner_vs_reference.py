@@ -7,8 +7,12 @@ execution_result.h, bound by bind.cpp).
   ``PipelineTemplateGenerator.create_pipeline_templates`` returns and the rank grid of each.  This repo's template search
   (csrc/planning/template_search.cpp behind ``oob_plan_pipeline_templates``) and ``PipelineTemplate.get_rank_grid`` must
   reproduce them: same stage boundaries, same GPUs per stage, iteration time to 1e-12, rank grids equal.
-* when oracle/_ref holds the built module (this container), the same comparison runs live on further random profiles,
-  and the reference's own planner tests (tests/planning/test_pipeline_template.py:10-100) run against both modules.
+* ``tests/golden/planner_more.json`` (``gen_planner_golden.py --more``, from the same module) holds further comparisons:
+  rank grids of 60 hand-built templates, the templates for 24 more random profiles, stage objects built the reference's
+  way, and what the reference's ``get_profile_results`` read back from a profile this package's ``save_profile_results``
+  wrote.
+* when oracle/_ref holds the built module, the reference's own planner tests (tests/planning/test_pipeline_template.py:
+  10-100) run against both modules.
 """
 import importlib
 import json
@@ -22,9 +26,11 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests", "golden"))
 
+from gen_planner_golden import results_from_rows  # noqa: E402
 from oobleck_b200.planning import pipeline_template as P  # noqa: E402
 
 GOLDEN = json.load(open(os.path.join(ROOT, "tests", "golden", "planner.json")))
+MORE = json.load(open(os.path.join(ROOT, "tests", "golden", "planner_more.json")))
 
 
 def reference_module():
@@ -38,17 +44,6 @@ def reference_module():
         return None
     finally:
         sys.path.remove(d)
-
-
-def results_from_rows(mod, rows):
-    return mod.LayerExecutionResults([
-        mod.LayerExecutionResult(i, r["forward"], r["backward"], {int(k): v for k, v in r["allreduce_in_node"].items()},
-                                 {int(k): v for k, v in r["allreduce_across_nodes"].items()}, tuple(r["mem_required"]))
-        for i, r in enumerate(rows)])
-
-
-def shape(t):
-    return t._num_nodes, [(list(s._layer_indices), s._num_gpus) for s in t.get_stages()]
 
 
 @pytest.mark.parametrize("case", GOLDEN, ids=[f"seed{c['seed']}-{c['layers']}L-{c['gpus_per_node']}gpn" for c in GOLDEN])
@@ -72,52 +67,25 @@ def test_template_search_reproduces_the_reference_planner(case):
 
 def test_rank_grid_of_hand_built_templates_matches_the_reference_module():
     """pipeline_template.h:57-84 directly (before: pinned only through the reference's test tables)."""
-    R = reference_module()
-    if R is None:
-        pytest.skip("oracle/_ref not built (make -C oracle needs /root/reference)")
-    rnd = random.Random(5)
-    for _ in range(60):
-        gpn = rnd.choice([1, 2, 4, 8])
-        nodes = rnd.randint(1, 4)
-        # stages: every node's GPUs are dealt out in power-of-two pieces
-        gpus = []
-        for _n in range(nodes):
-            left = gpn
-            while left:
-                g = rnd.choice([x for x in (1, 2, 4, 8) if x <= left])
-                gpus.append(g)
-                left -= g
-        layers = len(gpus) + rnd.randint(0, 6)
-        cuts = sorted(rnd.sample(range(1, layers), len(gpus) - 1)) if len(gpus) > 1 else []
-        bounds = list(zip([0] + cuts, cuts + [layers]))
-        rows = [{"forward": 1.0, "backward": 2.0, "allreduce_in_node": {str(g): 0.1 for g in range(1, 9)},
-                 "allreduce_across_nodes": {"1": 0.1}, "mem_required": [8, 8]} for _ in range(layers)]
-        rprof = results_from_rows(R, rows)
-        rt = R.PipelineTemplate([R.StageExecutionResult(rprof, (a, b), g) for (a, b), g in zip(bounds, gpus)], 1.0,
-                                layers, nodes, gpn)
-        mt = P.PipelineTemplate([P.StageExecutionResult(range(a, b), g) for (a, b), g in zip(bounds, gpus)], 1.0,
-                                layers, nodes, gpn)
-        ranks = rnd.sample(range(1000), sum(gpus))
-        assert mt.get_rank_grid(ranks) == rt.get_rank_grid(ranks)
+    from gen_planner_golden import hand_built_templates
+    cases = hand_built_templates()
+    assert len(cases) == len(MORE["rank_grids"]) == 60
+    for c, want in zip(cases, MORE["rank_grids"]):
+        mt = P.PipelineTemplate([P.StageExecutionResult(range(a, b), g) for (a, b), g in zip(c["bounds"], c["gpus"])],
+                                1.0, c["layers"], c["nodes"], c["gpus_per_node"])
+        assert {str(k): v for k, v in mt.get_rank_grid(c["ranks"]).items()} == want
 
 
 @pytest.mark.parametrize("seed", range(100, 124))
 def test_live_comparison_on_random_profiles(seed):
-    R = reference_module()
-    if R is None:
-        pytest.skip("oracle/_ref not built (make -C oracle needs /root/reference)")
-    from gen_planner_golden import profile_rows
-    rnd = random.Random(seed)
-    gpn = rnd.choice([1, 1, 2, 4])
-    layers = rnd.randint(3, 11)
-    lo = rnd.randint(1, 3)
-    hi = rnd.randint(lo, min(layers, lo + 4))
-    rows = profile_rows(seed, layers, gpn, rnd.choice([1, 1, 10, 40]))
-    theirs = R.PipelineTemplateGenerator().create_pipeline_templates(results_from_rows(R, rows), (lo, hi), gpn)
-    mine = P.PipelineTemplateGenerator().create_pipeline_templates(results_from_rows(P, rows), (lo, hi), gpn)
-    assert [shape(t) for t in mine] == [shape(t) for t in theirs]
-    for a, b in zip(mine, theirs):
-        assert a._iteration_time == pytest.approx(b._iteration_time, rel=1e-12)
+    from gen_planner_golden import RANDOM_PROFILE_SEEDS, random_profile_case, template_shape
+    theirs = MORE["random_profiles"][RANDOM_PROFILE_SEEDS.index(seed)]
+    assert theirs["seed"] == seed
+    gpn, node_range, rows = random_profile_case(seed)
+    mine = P.PipelineTemplateGenerator().create_pipeline_templates(results_from_rows(P, rows), node_range, gpn)
+    assert [template_shape(t) for t in mine] == theirs["shapes"]
+    for a, b in zip(mine, theirs["iteration_times"]):
+        assert a._iteration_time == pytest.approx(b, rel=1e-12)
 
 
 # ---- the reference's own planner tests (tests/planning/test_pipeline_template.py:10-100), on both modules ---------------
@@ -204,19 +172,16 @@ def test_create_pipeline_templates_multiple_gpus_in_node_range(planner):
 
 def test_stage_objects_built_the_references_way_agree():
     """``StageExecutionResult(layer_results, (begin, end), num_gpus)`` (bind.cpp:40-48): same aggregates on both sides."""
-    R = reference_module()
-    if R is None:
-        pytest.skip("oracle/_ref not built (make -C oracle needs /root/reference)")
-    from gen_planner_golden import profile_rows
+    from gen_planner_golden import STAGE_OBJECT_BOUNDS, profile_rows
     rows = profile_rows(3, 9, 4)
-    for begin, end, gpus in [(0, 9, 1), (2, 5, 2), (4, 9, 4), (0, 1, 1)]:
+    for (begin, end, gpus), b in zip(STAGE_OBJECT_BOUNDS, MORE["stage_objects"], strict=True):
         a = P.StageExecutionResult(results_from_rows(P, rows), (begin, end), gpus)
-        b = R.StageExecutionResult(results_from_rows(R, rows), (begin, end), gpus)
-        assert a._layer_indices == list(b._layer_indices) and a._num_gpus == b._num_gpus
-        assert a._num_layers == b._num_layers == end - begin
-        assert a._forward == pytest.approx(b._forward, rel=1e-15) and a._backward == pytest.approx(b._backward, rel=1e-15)
-        assert a._mem_required == b._mem_required
-    assert results_from_rows(P, rows).size == results_from_rows(R, rows).size == 9
+        assert a._layer_indices == b["layer_indices"] and a._num_gpus == b["num_gpus"]
+        assert a._num_layers == b["num_layers"] == end - begin
+        assert a._forward == pytest.approx(b["forward"], rel=1e-15)
+        assert a._backward == pytest.approx(b["backward"], rel=1e-15)
+        assert a._mem_required == b["mem_required"]
+    assert results_from_rows(P, rows).size == MORE["stage_objects_profile_size"] == 9
     assert results_from_rows(P, rows).size() == 9          # the stub file's spelling (pipeline_template.pyi:21)
 
 
@@ -233,24 +198,24 @@ def test_golden_bookkeeping_vectors_reproduce_with_the_references_own_planner_ob
     assert r.returncode == 0 and "all golden files reproduced" in r.stderr, r.stderr[-2000:]
 
 
-def test_saved_profile_is_what_the_references_get_profile_results_reads():
+def test_saved_profile_is_what_the_references_get_profile_results_reads(tmp_path):
     """planning/profiler.py::save_profile_results -> the reference's C++ ``get_profile_results`` (it reads
-    /tmp/oobleck/profiles/<model>-<tag>/, pipeline_template.cpp:26-79)."""
-    R = reference_module()
-    if R is None:
-        pytest.skip("oracle/_ref not built (make -C oracle needs /root/reference)")
-    from gen_planner_golden import profile_rows
-    from oobleck_b200.planning.profiler import save_profile_results
-    rows = profile_rows(21, 7, 4)
-    mine = results_from_rows(P, rows)
-    tag = "b200_saved_profile_test"
-    directory = save_profile_results(mine, "gpt2", tag, 3)
-    assert str(directory) == f"/tmp/oobleck/profiles/gpt2-{tag}"
-    back = R.get_profile_results("gpt2", tag, 3)
-    assert back.size == mine.size == 7
-    for a, b in zip(mine.get(), back.get()):
-        assert b._index == a._index
-        assert b._forward == a._forward and b._backward == a._backward            # JSON round-trips doubles exactly
-        assert dict(b._allreduce_in_node) == a._allreduce_in_node
-        assert dict(b._allreduce_across_nodes) == a._allreduce_across_nodes
-        assert tuple(b._mem_required) == a._mem_required
+    /tmp/oobleck/profiles/<model>-<tag>/, pipeline_template.cpp:26-79): the files written must be those the reference
+    read back, and what it read back must be this profile."""
+    from gen_planner_golden import SAVED_PROFILE, profile_rows
+    from oobleck_b200.planning.profiler import get_profile_path, save_profile_results
+    seed, layers, gpn, name, tag, mb = SAVED_PROFILE
+    mine = results_from_rows(P, profile_rows(seed, layers, gpn))
+    assert str(get_profile_path(name, tag)) == f"/tmp/oobleck/profiles/{name}-{tag}"
+    directory = save_profile_results(mine, name, tag, mb, cache=str(tmp_path))
+    assert directory == tmp_path / f"{name}-{tag}"
+    want = MORE["saved_profile"]
+    assert {f: json.load(open(directory / f)) for f in sorted(os.listdir(directory))} == want["files"]
+    back = want["read_back"]
+    assert len(back) == mine.size == 7
+    for a, b in zip(mine.get(), back):
+        assert b["index"] == a._index
+        assert b["forward"] == a._forward and b["backward"] == a._backward            # JSON round-trips doubles exactly
+        assert b["allreduce_in_node"] == {str(k): v for k, v in a._allreduce_in_node.items()}
+        assert b["allreduce_across_nodes"] == {str(k): v for k, v in a._allreduce_across_nodes.items()}
+        assert tuple(b["mem_required"]) == a._mem_required
